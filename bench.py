@@ -22,6 +22,9 @@ and comes out admitted or rejected, with the result of the SEQUENTIAL priority-o
 --config C4X  the part of the path that DOES shard: the score pass (K1 + K2) on a cluster 4x C4, node-range shards, one rank per
               GPU, ONE all-reduce of per-shard feasibility / capacity counts (NCCL); strong scaling, pairs scored per second.
 --config C5   steady-state churn (BASELINE.json config 5); C1..C3 the smaller configurations.
+--dump-outputs DIR   C1..C4 on the GPU: after the timed steps, what the last one computed (placements, gang status, scope
+              domains, committed node table; rank 0's cluster) goes to DIR as one float64 .npy per field.  The inputs are
+              seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -113,6 +116,25 @@ def workload_desc(name, n_nodes, n_gangs, n_cliques, n_gpus):
             "semantics": "sequential pass in (priority desc, submission index asc) order",
             "parallelism": "1 cluster on 1 GPU" if n_gpus == 1 else f"replicas only: {n_gpus} independent clusters, one per GPU",
             "l2": "inputs change every step (node table reset, claims rebuilt); the 126 MB L2 holds the working set by design"}
+
+
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, tables):
+    """every field of the result tables as DIR/<table>.<field>.npy in float64 (exact: the fields are integers below 2**53);
+    a table whose fields would exceed its share of DUMP_BYTES is cut to a fixed, seeded sample of its rows, whose indices
+    go to DIR/<table>.rows.npy"""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(tables)
+    for name, a in tables.items():
+        row_bytes = 8 * (1 + sum(int(np.prod(a.dtype[f].shape)) for f in a.dtype.names))
+        if len(a) * row_bytes > share:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), share // row_bytes, replace=False))
+            a = a[rows]
+            np.save(os.path.join(out_dir, f"{name}.rows.npy"), rows.astype(np.float64))
+        for f in a.dtype.names:
+            np.save(os.path.join(out_dir, f"{name}.{f}.npy"), a[f].astype(np.float64))
 
 
 def prefix_sample(g, c, s, keep):
@@ -259,6 +281,9 @@ def run_gpu(args):
         evals += st["evaluations"]
     sync()
     dt = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"placements": eng.placements(), "gang_status": eng.gang_status(),
+                                         "scope_domains": eng.scope_domains(), "nodes": eng.nodes()})
     # e2e through the C ABI with host buffers
     for _ in range(max(1, args.warmup // 2)):
         step_e2e()
@@ -524,7 +549,12 @@ def main():
     ap.add_argument("--config", default="C4", choices=sorted(synth.CONFIGS) + ["C5", "C4X"])
     ap.add_argument("--impl", default="grove_b200", choices=["grove_b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.config in ("C5", "C4X")):
+        ap.error("--dump-outputs covers the single-cycle lines on the GPU (C1-C4, --impl grove_b200)")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         if args.config == "C4X":
