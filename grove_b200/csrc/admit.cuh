@@ -695,6 +695,7 @@ __global__ void __launch_bounds__(128) k_shape_plaus(Topo tp, Tables tb, Relax r
   __shared__ uint32_t s_bits;
   const uint32_t shape = blockIdx.y, l = blockIdx.z;
   const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5, slot = threadIdx.x & 3u;
+  pdl_begin();
   const uint32_t gi = shape_rep[shape];
   const grove_gang_t gg = tb.gangs[gi];
   // candidate levels of the shape: Preferred (if any) down to Required; the whole cluster needs no table
@@ -739,37 +740,51 @@ __device__ __forceinline__ uint32_t eval_list_at(const Relax& rx, const Tables& 
   return tb.by_rank[rx.ctl[kEntryLo] + (i - nh - nl)];
 }
 
-// K3 launch forms: kW warps share ONE gang.  The candidates of the gang's level are pre-filtered 1024 at a time by all
+// K3 evaluators: kW warps share ONE gang.  The candidates of the gang's level are pre-filtered 1024 at a time by all
 // warps (a lane each); the plausible ones are then attempted kW at a time, a warp each, and the lowest successful
 // candidate IN ORDER is the answer -- exactly what trying them one after the other gives, minus the waiting.  kW = 1
-// while a round has many gangs (what matters is gangs in flight), 4 / 8 when it has few (what matters is the
+// while a round has many gangs (what matters is gangs in flight), 8 when it has few (what matters is the
 // latency of the slowest gang: a round lasts as long as its slowest evaluation).
-// Two launches per round, side by side on two streams: the LIGHT gangs (the tail of the list: most gangs, answered by their
+// Two roles in one launch per round (k_eval below): the LIGHT gangs (the tail of the list: most gangs, answered by their
 // first or second candidate) a warp each -- every resident warp does useful work --, the HEAVY ones (the head: gangs whose
 // last evaluation needed many attempts) kW warps each.  A light evaluation that is still unanswered after `max_att` attempts
 // gives up (kEvalDeferred): the gang stays dirty and comes back as a heavy one next round, instead of holding the round up.
 // Writes the "nxt" scratch of the gang.
 constexpr uint32_t kEvalDeferred = 0xFFu;   // nxt_tstate: no result this round
 constexpr int kHeavyWarps = 8;
+// the shared state of one evaluator
+template <int kW>
+struct EvalShared {
+  GangShared shs[kW];
+  int4 s_view[kW][kStageMax];
+  uint32_t s_vflag[kW][kStageMax];
+  alignas(16) uint8_t s_rk[kW][kStageMax + 256];
+  uint32_t s_plaus[32];                 // plausible candidates of the current 1024-candidate chunk, in order
+  uint32_t s_cl[kW][32], s_ch[kW][32];  // node ranges of the first chunk's candidates (kW runs of 32)
+  uint32_t s_win, s_ext, s_att, s_npl;
+};
+constexpr uint32_t kEvalThreads = kHeavyWarps * 32;
+constexpr size_t kEvalSmem = sizeof(EvalShared<kHeavyWarps>) > kHeavyWarps * sizeof(EvalShared<1>) ? sizeof(EvalShared<kHeavyWarps>)
+                                                                                                    : kHeavyWarps * sizeof(EvalShared<1>);
+
+// the barrier of one evaluator: the CTA for the heavy role, the warp for the light one (its warps finish different numbers of gangs)
+template <int kW>
+__device__ __forceinline__ void group_sync() {
+  if constexpr (kW == 1) __syncwarp(); else __syncthreads();
+}
+
 template <bool kPref, int kW, bool kHeavy>
-__global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tables tb, Relax rx, uint32_t max_att) {
-  __shared__ GangShared shs[kW];
-  __shared__ int4 s_view[kW][kStageMax];
-  __shared__ uint32_t s_vflag[kW][kStageMax];
-  __shared__ __align__(16) uint8_t s_rk[kW][kStageMax + 256];
-  __shared__ uint32_t s_plaus[32];   // plausible candidates of the current 1024-candidate chunk, in order
-  __shared__ uint32_t s_cl[kW][32], s_ch[kW][32];   // node ranges of the first chunk's candidates (kW runs of 32)
-  __shared__ uint32_t s_win, s_ext, s_att, s_npl;
-  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+__device__ __forceinline__ void eval_role(const Topo& tp, const Tables& tb, const Relax& rx, uint32_t max_att, EvalShared<kW>& es,
+                                          uint32_t slot, uint32_t n_slots) {
+  const uint32_t lane = threadIdx.x & 31, warp = kW == 1 ? 0u : threadIdx.x >> 5, tid = warp * 32 + lane;
   const uint32_t n_eval = rx.ctl[kNEval], n_heavy = rx.ctl[kNHeavy];
-  if (rx.ctl[kDone]) return;
-  GangShared& sh = shs[warp];
+  GangShared& sh = es.shs[warp];
   const uint32_t seg_lo = kHeavy ? 0u : n_heavy, seg_hi = kHeavy ? n_heavy : n_eval;
-  for (uint32_t ei = seg_lo + blockIdx.x; ei < seg_hi; ei += gridDim.x) {
+  for (uint32_t ei = seg_lo + slot; ei < seg_hi; ei += n_slots) {
     const uint32_t gi = eval_list_at(rx, tb, ei);
     const grove_gang_t gg = tb.gangs[gi];
     const GangInfo info = tb.ginfo[gi];
-    __syncthreads();   // the previous gang's shared state is no longer read
+    group_sync<kW>();   // the previous gang's shared state is no longer read
     // the gang's cliques and scopes (a lane each), the words of the re-evaluation shortcut and the base gang's rank are asked for
     // BEFORE anything looks at them: one L2 round trip for all of them instead of one per question
     const bool has_c = lane < gg.n_cliques, has_s = lane < gg.n_scopes;
@@ -789,10 +804,10 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
       if (bs != GROVE_GANG_ADMITTED) trivial = GROVE_GANG_BASE_REJECTED;
     }
     if (trivial) {
-      if (threadIdx.x == 0) {
+      if (tid == 0) {
         rx.nxt_tstate[gi] = uint8_t(trivial); rx.nxt_n[gi] = 0; rx.nxt_info[gi] = 0xFFu; rx.nxt_glo[gi] = GROVE_NONE_U32; rx.nxt_extent[gi] = 0;
       }
-      for (uint32_t si = threadIdx.x; si < gg.n_scopes; si += kW * 32) { rx.nxt_sc_lvl[gg.scope_off + si] = 0xFFu; rx.nxt_sc_lo[gg.scope_off + si] = GROVE_NONE_U32; }
+      for (uint32_t si = tid; si < gg.n_scopes; si += kW * 32) { rx.nxt_sc_lvl[gg.scope_off + si] = 0xFFu; rx.nxt_sc_lo[gg.scope_off + si] = GROVE_NONE_U32; }
       continue;
     }
     GangRegs g;
@@ -812,17 +827,17 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
       sh.Hlo[c] = 0; sh.Hhi[c] = 0; sh.c_got[c] = -1;
     }
     if (has_s) { sh.scopes[lane] = sc0; sh.s_got[lane] = -1; sh.s_lo[lane] = 0; }
-    if (threadIdx.x == 0) { s_win = GROVE_NONE_U32; s_ext = 0; s_att = 0; s_npl = 0; }
-    __syncthreads();
+    if (tid == 0) { es.s_win = GROVE_NONE_U32; es.s_ext = 0; es.s_att = 0; es.s_npl = 0; }
+    group_sync<kW>();
     // A candidate that failed in the gang's last evaluation fails again unless a claim was withdrawn inside it since: views only
     // shrink otherwise (claims are added, settled claims move into the committed state).  So a re-evaluation skips the
     // candidates in front of its last answer that no withdrawal touched -- gangs that meet a nearly full cluster would
     // otherwise re-run dozens of failing attempts every round.  (Single candidate level only.)
     Ev<kPref> ev(tp, rx, sh, g, lane);                         // candidates of any size, node state from L2
-    EvS<kPref> evs(tp, rx, sh, g, lane, s_view[warp], s_vflag[warp], s_rk[warp]);         // candidates of <= kStageMax nodes, node state staged in shared memory
+    EvS<kPref> evs(tp, rx, sh, g, lane, es.s_view[warp], es.s_vflag[warp], es.s_rk[warp]);         // candidates of <= kStageMax nodes, node state staged in shared memory
     bool staged = false;  // the winning attempt ran on evs
     bool won = false;     // this warp holds the answer
-    bool done = false;    // CTA-uniform
+    bool done = false;    // uniform over the evaluator
     int g_got = -1; uint32_t g_lo = 0;
     const long long t0 = rx.dbg ? clock64() : 0;
     // candidate levels: the Preferred level first (if any), widened level by level up to the Required one
@@ -838,11 +853,11 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
         staged = false;
         if (warp == 0) {
           won = place_in(ev, gg.n_scopes, 0, tp.n, -1);
-          if (won) { g_got = -1; g_lo = 0; if (lane == 0) s_win = 0; }
-          if (lane == 0) s_att += 1;
+          if (won) { g_got = -1; g_lo = 0; if (lane == 0) es.s_win = 0; }
+          if (lane == 0) es.s_att += 1;
         }
-        __syncthreads();
-        done = s_win != GROVE_NONE_U32;
+        group_sync<kW>();
+        done = es.s_win != GROVE_NONE_U32;
       } else {
         // candidate domains of level gl in score order: up to kMaxPieces ranges of domain indices
         uint32_t r0[kMaxPieces], rcnt[kMaxPieces], D = 0;
@@ -877,7 +892,7 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
               } else {
                 plaus = gang_plausible(tp, rx, sh, gg.n_scopes, dl, dh, gl, d);
               }
-              if (base == 0) { s_cl[c][lane] = dl; s_ch[c][lane] = dh; }
+              if (base == 0) { es.s_cl[c][lane] = dl; es.s_ch[c][lane] = dh; }
               if (plaus && k < fu) {   // failed last time: worth another attempt only if somebody withdrew a claim in there since
                 bool again = false;
                 for (uint32_t w = dl >> 5; w <= (dh - 1u) >> 5; ++w) again |= __ldg(rx.rem_round + w) >= le;
@@ -885,63 +900,63 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
               }
             }
             const uint32_t b = __ballot_sync(kFull, plaus);
-            if (lane == 0) s_plaus[c] = b;
+            if (lane == 0) es.s_plaus[c] = b;
           }
-          __syncthreads();
+          group_sync<kW>();
           uint32_t total = 0;
-          for (uint32_t c = 0; c < nchunk; ++c) total += __popc(s_plaus[c]);
-          if (threadIdx.x == 0) s_npl += total;
+          for (uint32_t c = 0; c < nchunk; ++c) total += __popc(es.s_plaus[c]);
+          if (tid == 0) es.s_npl += total;
           // attempts: kW plausible candidates at a time, in order, a warp each
           // while a round has many gangs the very first candidate is attempted by one warp alone: it usually succeeds,
           // and the other warps' attempts would be thrown away
           for (uint32_t j0 = 0; j0 < total && !done; j0 += uint32_t(kW)) {
-            if (!kHeavy && max_att && s_att >= max_att) { gave_up = true; break; }   // CTA-uniform (read after a barrier)
+            if (!kHeavy && max_att && es.s_att >= max_att) { gave_up = true; break; }   // uniform over the evaluator (read after its barrier)
             const uint32_t j = j0 + warp;
             bool ok = false; uint32_t dl = 0, dh = 0;
             if (j < total) {
               uint32_t rem = j, c = 0;   // the j-th set bit of the bitmap
-              for (; c + 1 < nchunk; ++c) { const uint32_t pc = __popc(s_plaus[c]); if (rem < pc) break; rem -= pc; }
-              uint32_t w = s_plaus[c];
+              for (; c + 1 < nchunk; ++c) { const uint32_t pc = __popc(es.s_plaus[c]); if (rem < pc) break; rem -= pc; }
+              uint32_t w = es.s_plaus[c];
               for (uint32_t i = 0; i < rem; ++i) w &= w - 1;
               const uint32_t kl = __ffs(w) - 1, k = base + c * 32 + kl;
-              if (base == 0) { dl = s_cl[c][kl]; dh = s_ch[c][kl]; } else cand(k, dl, dh);
+              if (base == 0) { dl = es.s_cl[c][kl]; dh = es.s_ch[c][kl]; } else cand(k, dl, dh);
               staged = dh - dl <= kStageMax;
               ok = staged ? place_in(evs, gg.n_scopes, dl, dh, gl) : place_in(ev, gg.n_scopes, dl, dh, gl);
-              if (lane == 0) { atomicAdd(&s_att, 1u); if (ok) atomicMin(&s_win, j); }
+              if (lane == 0) { atomicAdd(&es.s_att, 1u); if (ok) atomicMin(&es.s_win, j); }
               if (ok) k_won = k;
             }
-            __syncthreads();
-            const uint32_t win = s_win;
+            group_sync<kW>();
+            const uint32_t win = es.s_win;
             if (win != GROVE_NONE_U32) { done = true; won = ok && win == j; if (won) { g_got = gl; g_lo = dl; } }
           }
-          __syncthreads();   // s_plaus is rewritten by the next chunk
+          group_sync<kW>();   // es.s_plaus is rewritten by the next chunk
         }
       }
     } while (kPref && !done && !gave_up && --gl >= gbase);
     // what any of the attempts may have read (attempts past the winner only widen it)
-    if (lane == 0) atomicMax(&s_ext, max(max(ev.ext, evs.ext), fu ? ext_word : 0u));   // skipped candidates were read by the last evaluation
-    __syncthreads();
-    if (threadIdx.x == 0) rx.last_att[gi] = uint8_t(gave_up ? 255u : min(254u, s_att));
+    if (lane == 0) atomicMax(&es.s_ext, max(max(ev.ext, evs.ext), fu ? ext_word : 0u));   // skipped candidates were read by the last evaluation
+    group_sync<kW>();
+    if (tid == 0) rx.last_att[gi] = uint8_t(gave_up ? 255u : min(254u, es.s_att));
     if (gave_up) {   // no result this round: k_apply keeps the gang dirty
-      if (threadIdx.x == 0) rx.nxt_tstate[gi] = uint8_t(kEvalDeferred);
+      if (tid == 0) rx.nxt_tstate[gi] = uint8_t(kEvalDeferred);
       continue;
     }
-    if (rx.dbg && threadIdx.x == 0) {
+    if (rx.dbg && tid == 0) {
       const uint32_t cyc = uint32_t(clock64() - t0);
-      rx.dbg[gi * 8 + 0] += 1; rx.dbg[gi * 8 + 1] += s_npl; rx.dbg[gi * 8 + 2] += s_att;
-      rx.dbg[gi * 8 + 3] = max(rx.dbg[gi * 8 + 3], cyc); rx.dbg[gi * 8 + 4] = cyc; rx.dbg[gi * 8 + 5] = s_att; rx.dbg[gi * 8 + 6] = s_npl; rx.dbg[gi * 8 + 7] = rx.ctl[kRound];
+      rx.dbg[gi * 8 + 0] += 1; rx.dbg[gi * 8 + 1] += es.s_npl; rx.dbg[gi * 8 + 2] += es.s_att;
+      rx.dbg[gi * 8 + 3] = max(rx.dbg[gi * 8 + 3], cyc); rx.dbg[gi * 8 + 4] = cyc; rx.dbg[gi * 8 + 5] = es.s_att; rx.dbg[gi * 8 + 6] = es.s_npl; rx.dbg[gi * 8 + 7] = rx.ctl[kRound];
       // warp 0's own phases, summed over the cycle: staging, sub-domain pre-filter, packing, attempts staged
       atomicAdd(rx.dbg + tb.G * 8 + 0, evs.t_stage); atomicAdd(rx.dbg + tb.G * 8 + 1, evs.t_pre); atomicAdd(rx.dbg + tb.G * 8 + 2, evs.t_pack);
       atomicAdd(rx.dbg + tb.G * 8 + 3, evs.n_stage); atomicAdd(rx.dbg + tb.G * 8 + 4, cyc); atomicAdd(rx.dbg + tb.G * 8 + 5, 1u);
       atomicAdd(rx.dbg + tb.G * 8 + 6, evs.t_st2); atomicAdd(rx.dbg + tb.G * 8 + 7, evs.t_st3);
     }
     if (!done) {
-      if (threadIdx.x == 0) {
+      if (tid == 0) {
         rx.last_eval[gi] = round_now; rx.fail_upto[gi] = kFull;   // every candidate failed
         rx.nxt_tstate[gi] = GROVE_GANG_REJECTED; rx.nxt_n[gi] = 0; rx.nxt_info[gi] = 0xFFu; rx.nxt_glo[gi] = GROVE_NONE_U32;
-        rx.nxt_extent[gi] = s_ext;
+        rx.nxt_extent[gi] = es.s_ext;
       }
-      for (uint32_t si = threadIdx.x; si < gg.n_scopes; si += kW * 32) { rx.nxt_sc_lvl[gg.scope_off + si] = 0xFFu; rx.nxt_sc_lo[gg.scope_off + si] = GROVE_NONE_U32; }
+      for (uint32_t si = tid; si < gg.n_scopes; si += kW * 32) { rx.nxt_sc_lvl[gg.scope_off + si] = 0xFFu; rx.nxt_sc_lo[gg.scope_off + si] = GROVE_NONE_U32; }
       continue;
     }
     if (!won) continue;   // warp-uniform: the winner finishes alone
@@ -981,8 +996,26 @@ __global__ void __launch_bounds__(kW * 32, kW == 1 ? 16 : 2) k_eval(Topo tp, Tab
       rx.nxt_tstate[gi] = GROVE_GANG_ADMITTED; rx.nxt_n[gi] = uint16_t(n_ent);
       rx.nxt_info[gi] = (g_got >= 0 ? uint32_t(g_got) : 0xFFu) | (num << 8) | (den << 20);
       rx.nxt_glo[gi] = g_got >= 0 ? g_lo : GROVE_NONE_U32;
-      rx.nxt_extent[gi] = max(max(ev.ext, evs.ext), s_ext);   // the surplus pass above may have read further
+      rx.nxt_extent[gi] = max(max(ev.ext, evs.ext), es.s_ext);   // the surplus pass above may have read further
     }
+  }
+}
+
+// One launch per round, 256-thread CTAs.  CTAs [0, heavy_ctas) take the heavy role: kHeavyWarps warps share a gang, the list is
+// read from its head.  The others take the light role: every warp is an evaluator of its own (grid-strided over the warps of the
+// light CTAs) with the max_att give-up.  Heavy CTAs have the low indices so that they are dispatched first.  The role is
+// uniform over the CTA; each role's shared state is carved out of one dynamic buffer of kEvalSmem bytes.
+template <bool kPref>
+__global__ void __launch_bounds__(kEvalThreads, 2) k_eval(Topo tp, Tables tb, Relax rx, uint32_t heavy_ctas, uint32_t max_att) {
+  extern __shared__ __align__(16) unsigned char eval_smem[];
+  pdl_begin();
+  if (rx.ctl[kDone]) return;
+  if (blockIdx.x < heavy_ctas) {
+    eval_role<kPref, kHeavyWarps, true>(tp, tb, rx, 0u, *reinterpret_cast<EvalShared<kHeavyWarps>*>(eval_smem), blockIdx.x, heavy_ctas);
+  } else {
+    const uint32_t warp = threadIdx.x >> 5;
+    eval_role<kPref, 1, false>(tp, tb, rx, max_att, reinterpret_cast<EvalShared<1>*>(eval_smem)[warp],
+                               (blockIdx.x - heavy_ctas) * kHeavyWarps + warp, (gridDim.x - heavy_ctas) * kHeavyWarps);
   }
 }
 

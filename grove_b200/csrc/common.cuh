@@ -160,4 +160,14 @@ __device__ __forceinline__ bool stamp_below(uint32_t s, uint32_t round, uint32_t
   return (s >> 24) == stamp_tag(round) && (s & 0xFFFFFFu) < rank;
 }
 
+// Programmatic dependent launch: the kernels of a cycle after k_reset are launched so that the next one's CTAs can be
+// resident before this one ends (engine.cu launch_pdl).  Every such kernel calls pdl_begin() before its first global load,
+// store or atomic: griddepcontrol.wait returns once the preceding grid has completed and its writes are visible (at once
+// when the preceding operation was not a dependent launch), so ordering stays transitive along the stream; the trigger
+// right after it lets the next kernel be scheduled.
+__device__ __forceinline__ void pdl_begin() {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+
 }  // namespace grove

@@ -12,6 +12,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <utility>
 #include <new>
 #include <numeric>
 #include <string>
@@ -112,7 +113,6 @@ struct grove_engine {
   std::string err;
   cudaStream_t stream = nullptr;
   cudaStream_t stream_score = nullptr;  // K2 runs beside the relaxation (they only share the fit data)
-  cudaStream_t stream_heavy = nullptr;  // the heavy gangs of a round are evaluated beside the light ones
   cudaEvent_t ev_fit = nullptr, ev_score = nullptr, ev_s0 = nullptr, ev_s1 = nullptr;
   cudaEvent_t ev_nodes_up = nullptr, ev_tables_up = nullptr;  // the last upload out of the pinned node staging buffer / gang tables
   cudaEvent_t ev[10]{};
@@ -183,11 +183,10 @@ struct grove_engine {
   uint32_t tune_warp_ctas = 4;     // CTAs per SM of the warp-per-gang bookkeeping kernels (apply / detect / settle)
   uint32_t tune_batch = 3;         // rounds enqueued between two looks at the control words (GROVE_TUNE_AHEAD=0 / GROVE_DEBUG_ADMIT)
   uint32_t tune_ahead = 3;         // rounds kept in the queue while the host follows the relaxation through host-mapped progress words
-  uint32_t tune_eval_ctas = 0;     // k_eval CTAs per SM
+  uint32_t tune_eval_ctas = 0;     // light k_eval warps per SM (0: 16)
   uint32_t tune_heavy_att = 4;     // a gang whose last evaluation made this many attempts is heavy: kW warps next time
   uint32_t tune_max_att = 3;       // a light (one-warp) evaluation gives up after this many attempts and comes back heavy
   uint32_t tune_heavy_ctas = 2;    // heavy-form CTAs per SM
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   bool tune_overlap = true;        // K2 on a second stream beside the relaxation (GROVE_TUNE_OVERLAP=0 serialises them, e.g. to time K2 alone)
   bool tune_score = false;         // K2 score matrix: false = materialised on request (grove_build_score_matrix / the row getters),
                                    // true = every cycle, on the second stream beside the relaxation
@@ -232,6 +231,19 @@ struct grove_engine {
   } while (0)
 
 static int32_t fail(grove_engine* e, int32_t code, const char* msg) { e->err = msg; return code; }
+
+// Launch with programmatic stream serialization: the kernel's CTAs may become resident while the kernel before it on the
+// stream is still running.  The kernel must call pdl_begin() (common.cuh) before it touches global memory.
+template <typename... P, typename... A>
+static cudaError_t launch_pdl(void (*kernel)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, A&&... args) {
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...);
+}
 
 // ---------------------------------------------------------------------------------------------
 // topology: sort by label path, tree-ify ids, domain ranges.  Host side; runs only when labels change.
@@ -411,11 +423,11 @@ int32_t grove_engine_create(const grove_config_t* cfg, grove_engine_t** out) {
   cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);  // the latency-bound relaxation gets the SMs first
   if (cudaStreamCreateWithPriority(&e->stream, cudaStreamNonBlocking, prio_hi) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
   if (cudaStreamCreateWithPriority(&e->stream_score, cudaStreamNonBlocking, prio_lo) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
-  if (cudaStreamCreateWithPriority(&e->stream_heavy, cudaStreamNonBlocking, prio_hi) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
+  if (cudaFuncSetAttribute(k_eval<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kEvalSmem)) != cudaSuccess ||
+      cudaFuncSetAttribute(k_eval<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kEvalSmem)) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
   if (cudaEventCreateWithFlags(&e->ev_fit, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&e->ev_score, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&e->ev_nodes_up, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&e->ev_tables_up, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&e->ev_upd, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreate(&e->ev_s0) != cudaSuccess || cudaEventCreate(&e->ev_s1) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
   for (auto& ev : e->ev) if (cudaEventCreate(&ev) != cudaSuccess) { delete e; return GROVE_ERR_CUDA; }
   if (e->h_ctl.ensure(kCtlWords) != cudaSuccess) { delete e; return GROVE_ERR_OOM; }
@@ -437,12 +449,9 @@ void grove_engine_destroy(grove_engine_t* e) {
   if (e->ev_nodes_up) cudaEventDestroy(e->ev_nodes_up);
   if (e->ev_tables_up) cudaEventDestroy(e->ev_tables_up);
   if (e->ev_upd) cudaEventDestroy(e->ev_upd);
-  if (e->ev_fork) cudaEventDestroy(e->ev_fork);
-  if (e->ev_join) cudaEventDestroy(e->ev_join);
   if (e->ev_score) cudaEventDestroy(e->ev_score);
   if (e->h_live) cudaFreeHost(e->h_live);
   if (e->stream_score) cudaStreamDestroy(e->stream_score);
-  if (e->stream_heavy) cudaStreamDestroy(e->stream_heavy);
   if (e->stream) cudaStreamDestroy(e->stream);
   delete e;
 }
@@ -883,16 +892,17 @@ static int32_t build_ginfo(grove_engine* e) {
   return GROVE_OK;
 }
 
+// words of the per-domain capacity sum / max tables (each): k_fit accumulates into them with atomics, so the kernel before it
+// (k_reset for the first build of a cycle, k_fold for the others) zeroes them
+static uint32_t cap_words(const grove_engine* e) { return e->n_sigs * e->cap_stride; }
+
 // capacity tables over the committed state: K1 fit bitmap for every signature, per-node capacities, per-domain sum / max
 static int32_t build_cap_tables(grove_engine* e, const Topo& tp, const Tables& tb, const Relax& rx) {
   if (!e->n_sigs) return GROVE_OK;
   dim3 gfit(e->Npad / 1024, std::min<uint32_t>((e->n_sigs + kFitTile - 1) / kFitTile, 65535u));
-  if (e->cap_stride) {   // k_fit accumulates the per-domain sums / maxima with atomics
-    CU_TRY(e, cudaMemsetAsync(e->d_capsum.p, 0, sizeof(uint32_t) * size_t(e->n_sigs) * e->cap_stride, e->stream));
-    CU_TRY(e, cudaMemsetAsync(e->d_capmax.p, 0, sizeof(uint32_t) * size_t(e->n_sigs) * e->cap_stride, e->stream));
-  }
-  k_fit<<<gfit, 1024, 0, e->stream>>>(tp, tb, e->d_F.p, e->d_cap8.p, e->cap_stride ? e->d_capsum.p : nullptr, e->cap_stride ? e->d_capmax.p : nullptr);
-  k_clear_stale<<<(e->Npad / 4 + 255) / 256, 256, 0, e->stream>>>(rx, e->Npad / 4);
+  CU_TRY(e, launch_pdl(k_fit, gfit, 1024, 0, e->stream, tp, tb, e->d_F.p, e->d_cap8.p, e->cap_stride ? e->d_capsum.p : nullptr,
+                       e->cap_stride ? e->d_capmax.p : nullptr));
+  CU_TRY(e, launch_pdl(k_clear_stale, (e->Npad / 4 + 255) / 256, 256, 0, e->stream, rx, e->Npad / 4));
   if (e->shape_tables) {   // the candidate pre-filter of every gang shape over every domain of its candidate levels
     // only the levels some shape takes its candidates from (Preferred down to Required): a CTA that has nothing to do still
     // costs its launch, and the unit level alone would be tens of thousands of them
@@ -903,11 +913,11 @@ static int32_t build_cap_tables(grove_engine* e, const Topo& tp, const Tables& t
       const int first = g.preferred != GROVE_LEVEL_NONE && int(g.preferred) > base ? int(g.preferred) : base;
       for (int l = std::max(base, 0); l <= first && l < int(e->L); ++l) mx = std::max(mx, e->n_dom[l]);
     }
-    if (mx) k_shape_plaus<<<dim3((mx + 31) / 32, e->n_shapes, e->L), 128, 0, e->stream>>>(tp, tb, rx, e->d_shape_rep.p);
+    if (mx) CU_TRY(e, launch_pdl(k_shape_plaus, dim3((mx + 31) / 32, e->n_shapes, e->L), 128, 0, e->stream, tp, tb, rx, e->d_shape_rep.p));
     e->launches += 1;
   }
   CU_TRY(e, cudaGetLastError());
-  e->launches += 3;
+  e->launches += 2;
   return GROVE_OK;
 }
 
@@ -950,7 +960,7 @@ static int32_t cycle_begin(grove_engine* e) {
     const uint32_t W = e->tune_window ? e->tune_window : std::max(G, 1u);
     const uint32_t E = e->tune_entry ? e->tune_entry : W;
     if (e->h_live) { std::memset(e->h_live, 0, sizeof(uint32_t) * kLiveWords); e->h_live[kLiveRound] = 1; }
-    k_reset<<<e->n_sm * 4, 256, 0, e->stream>>>(make_relax(e), G, S, N, e->words, std::min(G, std::min(W, E)));
+    k_reset<<<e->n_sm * 4, 256, 0, e->stream>>>(make_relax(e), G, S, N, e->words, std::min(G, std::min(W, E)), cap_words(e));
     CU_TRY(e, cudaGetLastError());
   }
   e->launches = 0; e->in_cycle = true; e->have_results = false; e->have_scopes = false;
@@ -966,10 +976,10 @@ static int32_t finish_cycle(grove_engine* e) {
   if (G) {
     const uint32_t ncta = (G + kFinThreads - 1) / kFinThreads;
     CU_TRY(e, cudaMemsetAsync(e->d_fin.p + ncta, 0, sizeof(uint32_t) * 4, e->stream));
-    k_fin_count<<<ncta, kFinThreads, 0, e->stream>>>(tb, rx, e->d_fin.p);
-    k_fin_scan<<<1, 1024, 0, e->stream>>>(e->d_fin.p, ncta, e->d_totals.p);
-    k_fin_status<<<ncta, kFinThreads, 0, e->stream>>>(tb, rx, e->d_fin.p, e->d_perm.p, e->d_status.p);
-    k_emit<<<(G * 32 + 255) / 256, 256, 0, e->stream>>>(tb, rx, e->d_perm.p, e->d_status.p, e->d_out.p, e->d_scope_status.p);
+    CU_TRY(e, launch_pdl(k_fin_count, ncta, kFinThreads, 0, e->stream, tb, rx, e->d_fin.p));
+    CU_TRY(e, launch_pdl(k_fin_scan, 1, 1024, 0, e->stream, e->d_fin.p, ncta, e->d_totals.p));
+    CU_TRY(e, launch_pdl(k_fin_status, ncta, kFinThreads, 0, e->stream, tb, rx, e->d_fin.p, e->d_perm.p, e->d_status.p));
+    CU_TRY(e, launch_pdl(k_emit, (G * 32 + 255) / 256, 256, 0, e->stream, tb, rx, e->d_perm.p, e->d_status.p, e->d_out.p, e->d_scope_status.p));
     CU_TRY(e, cudaGetLastError());
     e->launches += 4;
     CU_TRY(e, cudaMemcpyAsync(e->h_ctl.p, e->d_totals.p, sizeof(uint32_t) * 4, cudaMemcpyDeviceToHost, e->stream));
@@ -994,7 +1004,7 @@ static int32_t finish_cycle(grove_engine* e) {
 
 struct CycleGuard {   // every error exit of a cycle leaves the handle usable (ADVICE round 1: in_cycle stayed set)
   grove_engine* e; bool armed = true;
-  ~CycleGuard() { if (armed) { e->in_cycle = false; cudaStreamSynchronize(e->stream); cudaStreamSynchronize(e->stream_score); cudaStreamSynchronize(e->stream_heavy); } }
+  ~CycleGuard() { if (armed) { e->in_cycle = false; cudaStreamSynchronize(e->stream); cudaStreamSynchronize(e->stream_score); } }
 };
 
 int32_t grove_run_cycle(grove_engine_t* e, grove_cycle_stats_t* stats) {
@@ -1028,8 +1038,8 @@ int32_t grove_run_cycle(grove_engine_t* e, grove_cycle_stats_t* stats) {
     }
     CU_TRY(e, cudaEventRecord(e->ev[2], e->stream));
     const uint32_t W = rx.window;
-    const uint32_t per_sm = e->tune_eval_ctas ? e->tune_eval_ctas : 16u;
-    const uint32_t eval_ctas = std::max(1u, std::min(W, e->n_sm * per_sm));
+    const uint32_t per_sm = e->tune_eval_ctas ? e->tune_eval_ctas : 16u;   // light warps
+    const uint32_t light_ctas = (std::max(1u, std::min(W, e->n_sm * per_sm)) + kHeavyWarps - 1) / kHeavyWarps;
     const uint32_t heavy_ctas = std::max(1u, std::min(W, e->n_sm * e->tune_heavy_ctas));
     const uint32_t warp_ctas = std::max(1u, std::min((W * 32 + 255) / 256, e->n_sm * e->tune_warp_ctas));
     // Rounds are enqueued `batch` at a time without waiting: every kernel returns at once when the cycle is over, so the
@@ -1042,32 +1052,22 @@ int32_t grove_run_cycle(grove_engine_t* e, grove_cycle_stats_t* stats) {
         CU_TRY(e, cudaMemsetAsync(e->d_add_stamp.p, 0xFF, sizeof(uint32_t) * e->Npad, e->stream));
         CU_TRY(e, cudaMemsetAsync(e->d_rem_stamp.p, 0xFF, sizeof(uint32_t) * e->words, e->stream));
       }
-      // heavy gangs (head of the list) on the second stream, kHeavyWarps warps each; light gangs (tail) a warp each
-      CU_TRY(e, cudaEventRecord(e->ev_fork, e->stream));
-      CU_TRY(e, cudaStreamWaitEvent(e->stream_heavy, e->ev_fork, 0));
-      if (e->any_preferred) {
-        k_eval<true, kHeavyWarps, true><<<heavy_ctas, kHeavyWarps * 32, 0, e->stream_heavy>>>(tp, tb, rx, 0);
-        k_eval<true, 1, false><<<eval_ctas, 32, 0, e->stream>>>(tp, tb, rx, e->tune_max_att);
-      } else {
-        k_eval<false, kHeavyWarps, true><<<heavy_ctas, kHeavyWarps * 32, 0, e->stream_heavy>>>(tp, tb, rx, 0);
-        k_eval<false, 1, false><<<eval_ctas, 32, 0, e->stream>>>(tp, tb, rx, e->tune_max_att);
-      }
-      CU_TRY(e, cudaEventRecord(e->ev_join, e->stream_heavy));
-      CU_TRY(e, cudaStreamWaitEvent(e->stream, e->ev_join, 0));
-      k_apply<<<warp_ctas, 256, 0, e->stream>>>(tb, rx);
-      k_detect<<<warp_ctas, 256, 0, e->stream>>>(tp, tb, rx, e->tune_refresh);
-      e->launches += 4;
+      // heavy gangs (head of the list) kHeavyWarps warps each, light gangs (tail) a warp each: one launch, two roles
+      CU_TRY(e, launch_pdl(e->any_preferred ? k_eval<true> : k_eval<false>, heavy_ctas + light_ctas, kEvalThreads, kEvalSmem, e->stream,
+                           tp, tb, rx, heavy_ctas, e->tune_max_att));
+      CU_TRY(e, launch_pdl(k_apply, warp_ctas, 256, 0, e->stream, tb, rx));
+      CU_TRY(e, launch_pdl(k_detect, warp_ctas, 256, 0, e->stream, tp, tb, rx, e->tune_refresh));
+      e->launches += 3;
       ++next_round;
       return GROVE_OK;
     };
-    auto fold = [&]() -> int32_t {   // the final gangs' claims -> committed state (relax.cuh k_fold)
-      k_fold<<<warp_ctas, 256, 0, e->stream>>>(tb, rx, e->d_nres.p);
-      k_fold_mark<<<1, 1, 0, e->stream>>>(rx);
-      e->launches += 2;
-      CU_TRY(e, cudaGetLastError());
+    // the final gangs' claims -> committed state (relax.cuh k_fold); before a rebuild it also zeroes the capacity sums / maxima
+    auto fold = [&](bool rebuild) -> int32_t {
+      CU_TRY(e, launch_pdl(k_fold, warp_ctas, 256, 0, e->stream, tb, rx, e->d_nres.p, rebuild ? cap_words(e) : 0u));
+      e->launches += 1;
       return GROVE_OK;
     };
-    auto fold_and_rebuild = [&]() -> int32_t { int32_t r = fold(); return r ? r : build_cap_tables(e, tp, tb, rx); };
+    auto fold_and_rebuild = [&]() -> int32_t { int32_t r = fold(true); return r ? r : build_cap_tables(e, tp, tb, rx); };
     // Following the relaxation WITHOUT blocking calls: the last CTA of k_detect leaves (round, done, refresh, ...) in host-mapped
     // memory; the host keeps `ahead` rounds enqueued beyond the one that runs and adds one more each time it sees a round end
     // (or a table rebuild first, when the device asked for one).  The GPU never waits for the host; the only waste is the
@@ -1134,7 +1134,7 @@ int32_t grove_run_cycle(grove_engine_t* e, grove_cycle_stats_t* stats) {
       if (e->h_ctl.p[kOvfCount] > rx.ovf_cap) return fail(e, GROVE_ERR_LIMIT, "claim overflow pool exhausted");
       rounds = e->h_ctl.p[kRound] - 1;
     }
-    rc = fold(); if (rc) return rc;   // everything is final now: the committed state and the final states of the outputs
+    rc = fold(false); if (rc) return rc;   // everything is final now: the committed state and the final states of the outputs
     e->last.evaluations = e->h_ctl.p[kEvals];
   }
   CU_TRY(e, cudaEventRecord(e->ev[3], e->stream));

@@ -35,6 +35,7 @@ __global__ void __launch_bounds__(1024) k_fit(Topo tp, Tables tb, uint32_t* __re
   const uint32_t n_rows = tb.S;                            // every signature of the submission
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t node = blockIdx.x * 1024 + tid;           // npad is a multiple of 1024
+  pdl_begin();
   const uint4 r = __ldg(tp.nres + node);
   const uint4 dm = __ldg(tp.ndom + node);
   const uint32_t gpu = r.z & 0xFFFFu, pods = r.z >> 16;

@@ -32,8 +32,10 @@ namespace grove {
 
 // The state a cycle starts from, in ONE launch (it used to be two dozen memsets and a blocking upload of the control words: a tenth
 // of a millisecond of launch latencies in front of every cycle)
-__global__ void __launch_bounds__(256) k_reset(Relax rx, uint32_t G, uint32_t NS, uint32_t npad, uint32_t words, uint32_t hi0) {
+// (n_cap: words of the capacity sum / max tables, which the first k_fit accumulates into)
+__global__ void __launch_bounds__(256) k_reset(Relax rx, uint32_t G, uint32_t NS, uint32_t npad, uint32_t words, uint32_t hi0, uint32_t n_cap) {
   const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
+  for (uint32_t i = tid; i < n_cap; i += nt) { rx.capsum[i] = 0; rx.capmax[i] = 0; }
   const uint4 ones = make_uint4(kFull, kFull, kFull, kFull);
   for (size_t i = tid; i < size_t(npad) * kClaimSlots; i += nt) rx.claims[i] = ones;
   for (uint32_t i = tid; i < npad; i += nt) { rx.ctot[i] = make_int4(0, 0, 0, 0); rx.cmaxr[i] = 0; rx.ovf_head[i] = 0; rx.add_stamp[i] = kFull; }
@@ -143,6 +145,7 @@ __device__ __forceinline__ uint32_t run_length(const uint32_t* node, const uint1
 // one warp per evaluated gang: publish a changed result
 __global__ void __launch_bounds__(256) k_apply(Tables tb, Relax rx) {
   const uint32_t lane = threadIdx.x & 31;
+  pdl_begin();
   if (rx.ctl[kDone]) return;
   const uint32_t n_eval = rx.ctl[kNEval], round = rx.ctl[kRound];
   const uint32_t nw = (gridDim.x * blockDim.x) >> 5;
@@ -210,6 +213,7 @@ __global__ void __launch_bounds__(256) k_apply(Tables tb, Relax rx) {
 __global__ void __launch_bounds__(256) k_detect(Topo tp, Tables tb, Relax rx, uint32_t refresh_every) {
   __shared__ bool s_last;
   const uint32_t lane = threadIdx.x & 31;
+  pdl_begin();
   if (rx.ctl[kDone]) return;   // uniform over the grid: set only by the last CTA of an earlier launch
   const uint32_t front = rx.ctl[kFront], hi = rx.ctl[kHi], round = rx.ctl[kRound];
   const uint32_t rem_any = rx.ctl[kRemAny];
@@ -289,11 +293,15 @@ __global__ void __launch_bounds__(256) k_detect(Topo tp, Tables tb, Relax rx, ui
 
 // one warp per gang that became final since the last fold: its claims move into the committed state.  Not every round: the
 // claims of final gangs are as good as committed for everybody who ranks after them, so the fold runs before a capacity-table
-// rebuild (the tables are built from the committed state) and when the cycle ends; k_fold_mark then moves the marker.
-__global__ void __launch_bounds__(256) k_fold(Tables tb, Relax rx, uint4* nres) {
+// rebuild (the tables are built from the committed state) and when the cycle ends; its last CTA then moves the marker.
+// Before a rebuild (n_cap != 0) it also zeroes the capacity sum / max tables that k_fit accumulates into.
+__global__ void __launch_bounds__(256) k_fold(Tables tb, Relax rx, uint4* nres, uint32_t n_cap) {
+  __shared__ bool s_last;
   const uint32_t lane = threadIdx.x & 31;
+  pdl_begin();
   const uint32_t lo = rx.ctl[kFolded], hi = rx.ctl[kFront];
   const uint32_t nw = (gridDim.x * blockDim.x) >> 5;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_cap; i += gridDim.x * blockDim.x) { rx.capsum[i] = 0; rx.capmax[i] = 0; }
   for (uint32_t p = lo + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5); p < hi; p += nw) {
     const uint32_t g = tb.by_rank[p];
     const uint32_t t = rx.tstate[g];
@@ -313,12 +321,17 @@ __global__ void __launch_bounds__(256) k_fold(Tables tb, Relax rx, uint4* nres) 
       atomicOr(rx.nlive + (n >> 2), kStale << ((n & 3u) * 8u));   // the capacity tables no longer describe this node
     }
   }
+  // the last CTA moves the marker, once every CTA has read it (the counter is k_detect's: idle between its launches)
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(rx.ctl + kCtaDone, 1u) == gridDim.x - 1;
+  __syncthreads();
+  if (s_last && threadIdx.x == 0) { rx.ctl[kFolded] = hi; rx.ctl[kCtaDone] = 0; }
 }
-__global__ void k_fold_mark(Relax rx) { rx.ctl[kFolded] = rx.ctl[kFront]; }
 
 // after a capacity-table build: the tables describe every node again
 __global__ void k_clear_stale(Relax rx, uint32_t n_words) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  pdl_begin();
   if (i < n_words) rx.nlive[i] &= ~0x80808080u;
   if (i == 0) { rx.ctl[kTablesAt] = rx.ctl[kFront]; rx.ctl[kRefresh] = 0; rx.ctl[kFoldAny] = 0; }
 }
@@ -333,6 +346,7 @@ __global__ void __launch_bounds__(kFinThreads) k_fin_count(Tables tb, Relax rx, 
   __shared__ uint32_t s_w[32];
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t g = blockIdx.x * kFinThreads + tid;
+  pdl_begin();
   uint32_t cnt = 0, adm = 0, rej = 0;
   if (g < tb.G) {
     const uint8_t st = rx.state[g];
@@ -357,6 +371,7 @@ __global__ void __launch_bounds__(1024) k_fin_scan(uint32_t* cta_tot, uint32_t n
   __shared__ uint32_t s_w[32];
   __shared__ uint32_t s_run;
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  pdl_begin();
   if (tid == 0) s_run = 0;
   __syncthreads();
   for (uint32_t base = 0; base < n_cta; base += 1024) {
@@ -381,6 +396,7 @@ __global__ void __launch_bounds__(kFinThreads) k_fin_status(Tables tb, Relax rx,
   __shared__ uint32_t s_w[32];
   const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t g = blockIdx.x * kFinThreads + tid;
+  pdl_begin();
   uint32_t cnt = 0; uint8_t st = 0;
   if (g < tb.G) { st = rx.state[g]; if (st == GROVE_GANG_ADMITTED) cnt = rx.cur_n[g]; }
   const uint32_t incl = warp_incl_scan(cnt, lane);
@@ -407,6 +423,7 @@ __global__ void k_emit(Tables tb, Relax rx, const uint32_t* __restrict__ perm, c
                        grove_placement_t* out, grove_scope_status_t* scopes_out) {
   const uint32_t lane = threadIdx.x & 31;
   const uint32_t g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  pdl_begin();
   if (g >= tb.G) return;
   const grove_gang_status_t st = status[g];
   const grove_gang_t gg = tb.gangs[g];
